@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the batched voice path on B200, one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload svf|biquad|delay|mfcc] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload svf|biquad|delay|mfcc] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one block (1024 frames) of one bank: BASELINE.json configs[1] by default -- 1 Mi voices of
 maxiOsc::saw -> maxiSVF (low-pass mix), per-voice fp64 output materialised time-major in HBM. With N > 1
@@ -28,6 +28,10 @@ voices are independent, so the headline block has no collective at any N.
              -O2 parity build and an -O3 -march=x86-64-v3 build side by side; a reported baseline, not the target
 
 `--impl reference` times only that CPU leg with the same metric/config (rank 0; other ranks exit 0).
+`--dump-outputs DIR` writes what the headline's last timed step computed as DIR/<name>.npy (rank 0; a fixed, seeded sample of
+DUMP_COLUMNS voices or channels of each array, fewer for the spectral arrays). Inputs are seeded, so two builds run with the same
+arguments compare output for output. Every --workload dumps its outputs; `--impl reference` times the CPU reference only and refuses
+the flag.
 """
 import argparse
 import json
@@ -35,14 +39,18 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
-os.environ.setdefault("MXB_PATCH_CACHE", os.path.join(ROOT, ".mxb_cache"))      # compiled patch kernels stay inside the repository
+if "MXB_PATCH_CACHE" not in os.environ:     # patch kernels compiled at run time are cached in a directory removed at exit
+    _patch_cache = tempfile.TemporaryDirectory(prefix="mxb_patch_cache_")
+    os.environ["MXB_PATCH_CACHE"] = _patch_cache.name
 
 BLOCK = 1024
 SR = 48000
@@ -57,6 +65,20 @@ WORKLOADS = {
                   desc="configs[2]: 256Ki voices saw -> maxiEnv::adsr -> maxiDelayline::dl(4096), fp64 out materialised"),
 }
 CPU_BLOCKS_PER_STEP = 8       # the reference arm: one step = this many consecutive blocks of the CPU sample (32 for the delay chain)
+DUMP_COLUMNS = 4096           # --dump-outputs: voices (channels) kept per array; 4096 x 1024 frames of fp64 = 32 MiB
+
+
+def dump_output(E, args, name, t, dim=1, columns=DUMP_COLUMNS):
+    """--dump-outputs: device tensor `t`, the result of the last timed step, as DIR/<name>.npy; along `dim` (voices or channels) a
+    fixed, seeded sample of `columns` entries, in ascending order, when it has more."""
+    if not args.dump_outputs or E.rank != 0:
+        return
+    n = t.shape[dim]
+    if n > columns:
+        idx = np.sort(np.random.default_rng(0).choice(n, columns, replace=False))
+        t = t.index_select(dim, E.torch.from_numpy(idx).to(t.device))
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
 
 
 def load_peaks():
@@ -400,8 +422,8 @@ def max_over_ranks(E, x):
     return float(t.item())
 
 
-def bank_leg(E, args, wl_name, steps, warmup, want_mix=False, with_onbox=False, full_readback=False):
-    """One bank workload: resident-throughput, roofline and the pipelined e2e number."""
+def bank_leg(E, args, wl_name, steps, warmup, want_mix=False, with_onbox=False, full_readback=False, dump=False):
+    """One bank workload: resident-throughput, roofline and the pipelined e2e number. dump: --dump-outputs of the timed block."""
     torch, capi, W = E.torch, E.capi, E.W
     wl = WORKLOADS[wl_name]
     V = int(os.environ.get("MXB_BENCH_VOICES", wl["voices"]))      # experiment hook (wave-quantisation probes); the JSON states voices_per_gpu
@@ -446,6 +468,10 @@ def bank_leg(E, args, wl_name, steps, warmup, want_mix=False, with_onbox=False, 
     torch.cuda.synchronize()
     t_wall1 = time.perf_counter()
     barrier(E)
+    if dump:
+        dump_output(E, args, "out", out)
+        if want_mix:
+            dump_output(E, args, "mix", mix)
     launches = bank.launches - launches0
     ms_total = evs[0].elapsed_time(evs[-1])
     per_launch_ms = sorted(evs[i].elapsed_time(evs[i + 1]) for i in range(steps))
@@ -729,7 +755,7 @@ def cpu_baseline_mfcc(budget_s=3.0):
     return out
 
 
-def mfcc_leg(E, args, steps, warmup):
+def mfcc_leg(E, args, steps, warmup, dump=False):
     torch, capi, W = E.torch, E.capi, E.W
     rank, world, dev, stream = E.rank, E.world, E.dev, E.stream
     wl = MFCC_WL
@@ -758,6 +784,8 @@ def mfcc_leg(E, args, steps, warmup):
     torch.cuda.synchronize()
     tw1 = time.perf_counter()
     barrier(E)
+    if dump:
+        dump_output(E, args, "mfcc", coeffs, dim=0)
     ms = e0.elapsed_time(e1)
     ms_max = max_over_ranks(E, ms)
     frames_per_step = C * H
@@ -824,8 +852,9 @@ def _tables():
     return g["sine"], g["transition"], float(g["sine_before"])
 
 
-def cpu_patch_rate(kind, budget_s, voices=4096):
-    """the reference's own objects run the same stage list per sample (oracle/ref_shim.cpp), voices partitioned over pinned threads"""
+def cpu_patch_rate(kind, budget_s, voices=4096, blocks=None):
+    """the reference's own objects run the same stage list per sample (oracle/ref_shim.cpp), voices partitioned over pinned threads;
+    >= budget_s seconds timed (or exactly `blocks` blocks for the reference arm)"""
     from maximilian_b200 import workloads as W
     from oracle import oracle_py as O
     O.load(kind)
@@ -854,7 +883,9 @@ def cpu_patch_rate(kind, budget_s, voices=4096):
         return job
     farm.run(job_n(1, 0))
     n, total, per = 0, 0.0, 2
-    while total < budget_s and n < 1024:
+    if blocks is not None:
+        total, n = farm.run(job_n(blocks, 0)), blocks
+    while blocks is None and total < budget_s and n < 1024:
         dt = farm.run(job_n(per, n))
         total += dt; n += per
         if dt < budget_s / 4:
@@ -879,7 +910,7 @@ def cpu_baseline_patch(budget_s=3.0):
     return out
 
 
-def patch_leg(E, args, steps, warmup):
+def patch_leg(E, args, steps, warmup, dump=False):
     """The reference's polysynth example as a voice patch: the kernel generated + NVRTC-compiled for its stage list (K8f), the
     interpreting kernel (K8) beside it, and the e2e loop with the trigger bytes coming from the host every block."""
     torch, capi, W = E.torch, E.capi, E.W
@@ -933,6 +964,9 @@ def patch_leg(E, args, steps, warmup):
                                create_seconds=compile_s)
         if mode == "fused":
             t_wall = [tw0, tw1]
+            if dump:
+                dump_output(E, args, "out", out)
+                dump_output(E, args, "mix", mix[(warmup + n - 1) & 1])
     # ---- e2e: per step this block's trigger bytes go up from pinned memory on a copy stream (double-buffered on the device), the
     # fused patch runs, the stereo bus comes back into one of two pinned buffers; one synchronisation at the end
     pt = patches["fused"]
@@ -997,7 +1031,7 @@ SPEC_WL = dict(channels=1 << 14, fft=1024, hop=512, hops_per_step=8,
                     "analysis with maxiFFTOctaveAnalyzer (averages + peaks) and maxiBark (specific / relative / total loudness) fused in")
 
 
-def modulated_leg(E, args, steps, warmup):
+def modulated_leg(E, args, steps, warmup, dump=False):
     """SURVEY.md 8(f) rank 1, timed: the banks with a per-sample oscillator frequency (FM: `osc.saw(f + lfo)`, the reference takes the
     frequency by argument on every call) -- one more 8-byte stream READ per voice-sample, resident on the device like the output.
     fm_svf: configs[1]'s bank (K1, MOD instantiation); fm_delay: configs[2]'s bank (K2, the modulated instantiation of its windows)."""
@@ -1036,6 +1070,8 @@ def modulated_leg(E, args, steps, warmup):
             step()
         e1.record(stream)
         torch.cuda.synchronize()
+        if dump:
+            dump_output(E, args, key + "_out", out, columns=DUMP_COLUMNS // 2)
         ms = e0.elapsed_time(e1) / steps
         peak, peak_src = load_peaks()
         bytes_per = wl["bytes_per"] + 8.0
@@ -1054,9 +1090,10 @@ def modulated_leg(E, args, steps, warmup):
     return res
 
 
-def spectral_extra_leg(E, args, steps, warmup):
+def spectral_extra_leg(E, args, steps, warmup, dump=False):
     """The rows of SURVEY.md 8(f) around the transform that the MFCC leg does not touch: the full-spectrum analysis (cartToPol incl.
-    atan2), the octave-analyser / Bark epilogues, and maxiIFFT. Each sub-leg: CUDA events over `steps` steps, algorithmic bytes."""
+    atan2), the octave-analyser / Bark epilogues, and maxiIFFT. Each sub-leg: CUDA events over `steps` steps, algorithmic bytes.
+    dump: --dump-outputs of each sub-leg's last step, DUMP_COLUMNS / 8 channels (8 MiB per spectrum array)."""
     import ctypes as C_
     torch, capi, W = E.torch, E.capi, E.W
     dev, stream, world = E.dev, E.stream, E.world
@@ -1096,6 +1133,9 @@ def spectral_extra_leg(E, args, steps, warmup):
     # (1) analysis with the whole spectrum leaving the chip: magnitudes + phases (atan2f per bin)
     st = capi.Stft(C, n, hop, ctx=E.ctx)
     ms = timed(lambda: st.process_device(x.data_ptr(), H * hop, 1, H * hop, H, mags=mags.data_ptr(), phases=phases.data_ptr(), stream=stream.cuda_stream), steps)
+    if dump:
+        dump_output(E, args, "analysis_mags", mags, dim=0, columns=DUMP_COLUMNS // 8)
+        dump_output(E, args, "analysis_phases", phases, dim=0, columns=DUMP_COLUMNS // 8)
     out["analysis_mags_phases"] = entry(ms, hop * 4 + 2 * bins * 4, "stft_stream_kernel<FULL>", "maxiFFT::process + cartToPol, magnitudes and phases written")
     # (2) resynthesis: maxiIFFT SPECTRUM from those magnitudes / phases
     ist = capi.Istft(C, n, hop, ctx=E.ctx)
@@ -1103,6 +1143,8 @@ def spectral_extra_leg(E, args, steps, warmup):
     def resyn():
         capi.check(L.mxb_istft_process(ist.h, C_.c_void_p(mags.data_ptr()), C_.c_void_p(phases.data_ptr()), H, C_.c_void_p(y.data_ptr()), capi.MEM_DEVICE, sp), "mxb_istft_process")
     ms = timed(resyn, steps)
+    if dump:
+        dump_output(E, args, "resynthesis", y, dim=0, columns=DUMP_COLUMNS // 8)
     out["resynthesis"] = entry(ms, 2 * bins * 4 + hop * 4, "istft1024_kernel", "maxiIFFT::process(SPECTRUM): polToCart, inverse transform, window, overlap-add", "istft")
     del ist, y, phases
     # (3) analysis with the octave analyser and Bark loudness fused in (magnitudes written too)
@@ -1116,6 +1158,10 @@ def spectral_extra_leg(E, args, steps, warmup):
     def analyse():
         capi.check(L.mxb_stft_process3(st.h, C_.c_void_p(x.data_ptr()), H * hop, 1, H * hop, H, C_.byref(o), C_.byref(post), None, C_.byref(nf), capi.MEM_DEVICE, sp), "mxb_stft_process3")
     ms = timed(analyse, steps)
+    if dump:
+        for name, t in (("octave_bark_mags", mags), ("octave_averages", av), ("octave_peaks", pk), ("bark_specific", bs), ("bark_relative", br),
+                        ("bark_total", bt)):
+            dump_output(E, args, name, t, dim=0, columns=DUMP_COLUMNS // 8)
     out["analysis_octave_bark"] = entry(ms, hop * 4 + bins * 4 + 2 * nA * 4 + (48 + 1) * 8, "stft_stream_kernel<FULL> + octave / Bark epilogues",
                                         f"maxiFFT::process + maxiFFTOctaveAnalyzer::calculate ({nA} averages, peaks) + maxiBark, magnitudes written")
     out["config"] = {"workload": wl["desc"], "channels_per_gpu": C, "hops_per_step": H}
@@ -1151,7 +1197,11 @@ def main():
     ap.add_argument("--f32-out", action="store_true", help="store the materialised output as fp32 (declared in the JSON)")
     ap.add_argument("--collective", default="p2p", choices=["p2p", "nccl"],
                     help="N > 1 mix-down: p2p = peer-memory exchange fused into the mix-reduce kernel (default); nccl = torch.distributed all_reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step computed as DIR/<name>.npy (a fixed, seeded sample of voices or channels)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference only times the CPU reference")
     extras_wanted = args.workload is None and not args.no_extras
     wl_name = args.workload or "svf"
     if args.impl == "reference":
@@ -1164,19 +1214,19 @@ def main():
     E = setup_env(args)
 
     if wl_name == "spectral":
-        r = spectral_extra_leg(E, args, max(3, min(args.steps, 20)), args.warmup)
+        r = spectral_extra_leg(E, args, args.steps, args.warmup, dump=True)
         if E.rank == 0:
             print(json.dumps({"metric": "fft_frames_per_sec", "unit": "frames/s", "n_gpus": E.world, "higher_is_better": True, "data": "synthetic", **r}), flush=True)
         return finish(E)
 
     if wl_name == "modulated":
-        r = modulated_leg(E, args, max(3, min(args.steps, 40)), args.warmup)
+        r = modulated_leg(E, args, args.steps, args.warmup, dump=True)
         if E.rank == 0:
             print(json.dumps({"metric": "voice_samples_per_sec", "unit": "samples/s", "n_gpus": E.world, "higher_is_better": True, "data": "synthetic", **r}), flush=True)
         return finish(E)
 
     if wl_name == "patch":
-        head = patch_leg(E, args, args.steps, args.warmup)
+        head = patch_leg(E, args, args.steps, args.warmup, dump=True)
         if E.rank == 0:
             line = {"metric": "voice_samples_per_sec", "value": head["value"], "unit": "samples/s", "n_gpus": E.world, "steps": args.steps,
                     "warmup": args.warmup, "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -1187,7 +1237,7 @@ def main():
         return finish(E)
 
     if wl_name == "mfcc":
-        head = mfcc_leg(E, args, args.steps, args.warmup)
+        head = mfcc_leg(E, args, args.steps, args.warmup, dump=True)
         if E.rank == 0:
             line = {"metric": "fft_mfcc_frames_per_sec", "value": head["value"], "unit": "frames/s", "n_gpus": E.world, "steps": args.steps,
                     "warmup": args.warmup, "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -1199,7 +1249,7 @@ def main():
         return finish(E)
 
     want_mix = args.mix == 1
-    head = bank_leg(E, args, wl_name, args.steps, args.warmup, want_mix=want_mix, with_onbox=True, full_readback=extras_wanted)
+    head = bank_leg(E, args, wl_name, args.steps, args.warmup, want_mix=want_mix, with_onbox=True, full_readback=extras_wanted, dump=True)
     mixdown = None
     if args.mix < 0 and not WORKLOADS[wl_name]["delay"]:
         mhz = E.torch.tensor([float((head.get("clocks") or {}).get("sm_mhz") or 0.0)], dtype=E.torch.float64, device=E.dev)
@@ -1266,7 +1316,7 @@ def reference_arm_patch(args):
     if int(os.environ.get("RANK", "0")) != 0:
         return
     kind = cpu_kinds()[-1]
-    v, voices, threads, n, dt = cpu_patch_rate(kind, 3.0 * max(1, min(args.steps, 10)) / 3.0)
+    v, voices, threads, n, dt = cpu_patch_rate(kind, None, blocks=args.steps)
     print(json.dumps({"impl": "reference", "metric": "voice_samples_per_sec", "value": v, "unit": "samples/s", "n_gpus": args.gpus, "steps": args.steps,
                       "warmup": 1, "ms_per_step": 1e3 * dt / max(1, n), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
                       "data": "synthetic", "config": {"workload": PATCH_WL["desc"], "cpu_sample_voices": voices, "block": BLOCK, "sample_rate": SR},

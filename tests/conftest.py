@@ -24,11 +24,27 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def reference():
-    """The unmodified reference compiled from /root/reference (absent on the GPU box unless prebuilt)."""
+def reference_traces():
+    """The stored reference traces, and the compiled reference where oracle/Makefile can build it or it was built before."""
+    import reference_trace
     from oracle import oracle_py
-    if os.path.isdir("/root/reference/src"):
-        oracle_py.build("reference")
-    if not oracle_py.available("reference"):
-        pytest.skip("oracle/_ref/libmaxiref.so not built and /root/reference absent")
-    return oracle_py
+    oracle_py.build("reference")                      # leaves oracle/_ref/ as it is where the reference sources are absent
+    store = reference_trace.Store()
+    yield store, (oracle_py if oracle_py.available("reference") else None)
+    store.save()
+
+
+@pytest.fixture
+def reference(request, port, reference_traces):
+    """The compiled reference's side of a bit-for-bit pin (tests/reference_trace.py): reference.check(run) compares run("port")
+    with the stored trace of run("reference"), and with a live run of the reference where it is built."""
+    import reference_trace
+    store, live = reference_traces
+    return reference_trace.Trace(reference_trace.key(request.node), store, live)
+
+
+@pytest.hookimpl(tryfirst=True)
+def pytest_collection_modifyitems(items):
+    """Every pinned test collected, before -k / -m deselect any: recording drops the stored traces of pins that no longer exist."""
+    import reference_trace
+    reference_trace.COLLECTED.update(reference_trace.key(it) for it in items if "reference" in getattr(it, "fixturenames", ()))

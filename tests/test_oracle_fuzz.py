@@ -1,7 +1,8 @@
 """Randomised pin of the plain-C oracle against the compiled reference: chains, sizes, sample rates and parameter
 values drawn from seeded generators -- including the ugly corners (zero / negative / above-Nyquist frequencies, duty
 outside [0, 1], resonance 0, hold times 0, one-slot delay lines, gates that open and close inside one block, modulated
-arguments) -- compared BIT FOR BIT over consecutive blocks, state included. CPU only; skipped without the reference.
+arguments) -- compared BIT FOR BIT over consecutive blocks, state included. CPU only; against the stored trace of the
+reference everywhere and the compiled reference itself where it is built (tests/reference_trace.py).
 """
 import numpy as np
 import pytest
@@ -12,10 +13,6 @@ OSCS = ["sinewave", "coswave", "phasor", "saw", "square", "pulse", "impulse", "t
 FILTS = ["none", "lores", "hires", "svf", "biquad"]
 BQ = ["lowpass", "highpass", "bandpass", "notch", "peak", "lowshelf", "highshelf"]
 RATES = [8000, 22050, 44100, 48000, 96000]
-
-
-def _same(a, b):
-    return np.array_equal(a, b, equal_nan=True)
 
 
 def _draw(seed):
@@ -48,58 +45,62 @@ def _draw(seed):
 
 @pytest.mark.parametrize("seed", range(60))
 def test_random_chain_bit_exact(port, reference, seed):
-    c, p, rng = _draw(seed)
-    V, B = c["V"], c["B"]
-    kw = dict(osc=c["osc"], filt=c["filt"], env=c["env"], delay=c["delay"], sample_rate=c["sr"], biquad_type=c["bq"],
-              svf_mix=tuple(float(m) for m in c["mix"]), delay_capacity=c["cap"])
-    a = port.Bank(V, kind="port", **kw); b = reference.Bank(V, kind="reference", **kw)
-    for bank in (a, b):
-        W.configure_bank(bank, c["filt"], p, bool(c["env"]), bool(c["delay"]), sample_rate=c["sr"])
+    def run(kind):
+        c, p, rng = _draw(seed)
+        V, B = c["V"], c["B"]
+        kw = dict(osc=c["osc"], filt=c["filt"], env=c["env"], delay=c["delay"], sample_rate=c["sr"], biquad_type=c["bq"],
+                  svf_mix=tuple(float(m) for m in c["mix"]), delay_capacity=c["cap"])
+        b = port.Bank(V, kind=kind, **kw)
+        W.configure_bank(b, c["filt"], p, bool(c["env"]), bool(c["delay"]), sample_rate=c["sr"])
         if c["delay"] == "position":
-            bank.set("delay_position", np.minimum(np.arange(V) * 2.0, c["cap"] - 1))
-    mod_ok = not c["env"] and not c["delay"]
-    for blk in range(3):
-        on = rng.integers(0, B + 1, V).astype(np.int32); off = rng.integers(0, B + 2, V).astype(np.int32)
-        kwp = {}
-        if mod_ok and blk == 1:
-            kwp["freq_tv"] = 50.0 + 2000.0 * rng.random((B, V))
-            if c["filt"] in ("lores", "hires", "svf"):
-                kwp["cutoff_tv"] = 30.0 + 0.4 * c["sr"] * rng.random((B, V))
-        if c["delay"] and blk == 1:
-            kwp["delay_size_tv"] = rng.integers(1, c["cap"] + 1, (B, V)).astype(np.float64)
-        oa, ma = a.process(B, on, off, want_mix=True, **kwp); ob, mb = b.process(B, on, off, want_mix=True, **kwp)
-        assert _same(oa, ob), (seed, c, blk)
-        assert _same(ma, mb), (seed, c, blk)
-    states = ["phase", "filt0", "filt1"] + (["filt2"] if c["filt"] == "svf" else [])
-    if c["env"]:
-        states += ["env_amplitude", "env_output", "env_holdcount", "env_flags"]
-    if c["delay"]:
-        states += ["delay_phase"]
-    for s in states:
-        assert _same(a.get(s), b.get(s)), (seed, c, s)
-    if c["delay"]:
-        for v in range(V):
-            assert _same(a.ring(v, c["cap"]), b.ring(v, c["cap"])), (seed, v)
+            b.set("delay_position", np.minimum(np.arange(V) * 2.0, c["cap"] - 1))
+        mod_ok = not c["env"] and not c["delay"]
+        for blk in range(3):
+            on = rng.integers(0, B + 1, V).astype(np.int32); off = rng.integers(0, B + 2, V).astype(np.int32)
+            kwp = {}
+            if mod_ok and blk == 1:
+                kwp["freq_tv"] = 50.0 + 2000.0 * rng.random((B, V))
+                if c["filt"] in ("lores", "hires", "svf"):
+                    kwp["cutoff_tv"] = 30.0 + 0.4 * c["sr"] * rng.random((B, V))
+            if c["delay"] and blk == 1:
+                kwp["delay_size_tv"] = rng.integers(1, c["cap"] + 1, (B, V)).astype(np.float64)
+            o, m = b.process(B, on, off, want_mix=True, **kwp)
+            yield f"out {blk} {c}", o
+            yield f"mix {blk} {c}", m
+        states = ["phase", "filt0", "filt1"] + (["filt2"] if c["filt"] == "svf" else [])
+        if c["env"]:
+            states += ["env_amplitude", "env_output", "env_holdcount", "env_flags"]
+        if c["delay"]:
+            states += ["delay_phase"]
+        for s in states:
+            yield f"{s} {c}", b.get(s)
+        if c["delay"]:
+            for v in range(V):
+                yield f"ring {v} {c}", b.ring(v, c["cap"])
+    reference.check(run)
 
 
 @pytest.mark.parametrize("seed", range(12))
 def test_random_spectral_bit_exact(port, reference, seed):
-    rng = np.random.default_rng(5000 + seed)
-    n = int(rng.choice([64, 128, 256, 512, 1024, 2048]))
-    hop = int(rng.choice([n // 8, n // 4, n // 2, n]))
-    C = int(rng.integers(1, 4))
-    x = W.channel_streams(C, int(rng.integers(n, 6 * n)), seed=seed)
-    x[0] *= float(rng.choice([1e-6, 1.0, 1e4]))
-    sa, sb = port.Stft(C, n, hop, kind="port"), reference.Stft(C, n, hop, kind="reference")
-    cuts = np.unique(np.r_[0, rng.integers(0, x.shape[1], 3), x.shape[1]])
-    for lo, hi in zip(cuts[:-1], cuts[1:]):
-        ra, rb = sa.process(x[:, lo:hi]), sb.process(x[:, lo:hi])
-        for k in ("mags", "phases", "re", "im"):
-            assert ra[k].shape == rb[k].shape and _same(ra[k], rb[k]), (seed, n, hop, k)
-    if n >= 128:
-        nf, nc = int(rng.integers(8, 43)), int(rng.integers(4, 41))
-        ma = port.Mfcc(n // 2, nf, nc, 20.0, 16000.0, 44100, kind="port"); mb = reference.Mfcc(n // 2, nf, nc, 20.0, 16000.0, 44100, kind="reference")
-        mags = port.Stft(1, n, hop, kind="port").process(x[:1])["mags"]
-        if mags.shape[1]:
-            (ca, ba), (cb, bb) = ma.process(mags), mb.process(mags)
-            assert _same(ca, cb) and _same(ba, bb), (seed, n, nf, nc)
+    def run(kind):
+        rng = np.random.default_rng(5000 + seed)
+        n = int(rng.choice([64, 128, 256, 512, 1024, 2048]))
+        hop = int(rng.choice([n // 8, n // 4, n // 2, n]))
+        C = int(rng.integers(1, 4))
+        x = W.channel_streams(C, int(rng.integers(n, 6 * n)), seed=seed)
+        x[0] *= float(rng.choice([1e-6, 1.0, 1e4]))
+        s = port.Stft(C, n, hop, kind=kind)
+        cuts = np.unique(np.r_[0, rng.integers(0, x.shape[1], 3), x.shape[1]])
+        for lo, hi in zip(cuts[:-1], cuts[1:]):
+            r = s.process(x[:, lo:hi])
+            for k in ("mags", "phases", "re", "im"):
+                yield f"{k} {lo}:{hi} (n {n}, hop {hop})", r[k]
+        if n >= 128:
+            nf, nc = int(rng.integers(8, 43)), int(rng.integers(4, 41))
+            mf = port.Mfcc(n // 2, nf, nc, 20.0, 16000.0, 44100, kind=kind)
+            mags = port.Stft(1, n, hop, kind="port").process(x[:1])["mags"]
+            if mags.shape[1]:
+                co, mb = mf.process(mags)
+                yield f"mfcc (n {n}, {nf} filters, {nc} coeffs)", co
+                yield f"melbands (n {n}, {nf} filters)", mb
+    reference.check(run)

@@ -1,6 +1,7 @@
 """Voice patches (include/maxib200.h mxb_patch; tests/patch_cases.py) on the CPU: the plain-C interpreter of oracle/maxi_oracle.c
 against the same stage lists run by the reference's own objects (oracle/ref_shim.cpp) -- bit for bit, outputs, buses and the state
-of every stage -- and against the committed fixture tests/golden/patches.npz where /root/reference is absent."""
+of every stage (live where the compiled reference is built, from its stored trace everywhere: tests/reference_trace.py) -- and
+against the committed fixture tests/golden/patches.npz."""
 import numpy as np
 import pytest
 
@@ -18,35 +19,42 @@ def _tables(port):
 
 def test_tables_fixture_is_the_references(port, reference):
     g = G.load("tables")
-    s, t, b = reference.get_tables("reference")
-    assert np.array_equal(s, g["sine"]) and np.array_equal(t, g["transition"]) and b == float(g["sine_before"])
-    assert s.size == 514 and t.size == 1001
+    assert g["sine"].size == 514 and g["transition"].size == 1001
+
+    def run(kind):
+        s, t, b = (g["sine"], g["transition"], float(g["sine_before"])) if kind == "port" else port.get_tables("reference")
+        yield "sine", s
+        yield "transition", t
+        yield "sine_before", b
+    reference.check(run)
 
 
 @pytest.mark.parametrize("case", PC.cases(), ids=lambda c: c[0])
 def test_patch_port_equals_reference(port, reference, case):
     name, d, params, inputs, exact, taps = case
     _tables(port)
-    V, B = 24, 200
-    po = port.Patch(d, V, delay_taps=taps, kind="port"); pr = reference.Patch(d, V, delay_taps=taps, kind="reference")
-    for k, v in params(V, 11).items():
-        po.set(k, v); pr.set(k, v)
-    for blk in range(3):
-        ins = inputs(V, B, blk, 7)
-        oo, mo = po.process(B, ins, want_mix=True); orr, mr = pr.process(B, ins, want_mix=True)
-        assert np.array_equal(oo, orr, equal_nan=True), (name, blk)
-        assert np.array_equal(mo, mr, equal_nan=True), (name, blk)
-        assert np.isfinite(orr).all() and np.abs(orr).max() > 1e-3
-    for si, (op, kind, dst, src) in enumerate(d.stages):
-        for sl in range(SLOTS.get(op, 0)):
-            if op == 5 and kind in (5, 6) and sl == 1:
-                continue                                   # lopass / hipass keep one value (outputs[0])
-            if op == 4 and sl == 3:
-                continue                                   # nxcHappened is indeterminate in the reference until the first trigger
-            assert np.array_equal(po.get_state(si, sl), pr.get_state(si, sl)), (name, si, sl)
-        if op in (10, 11):
-            for v in range(0, V, 5):
-                assert np.array_equal(po.ring(si, v, taps), pr.ring(si, v, taps)), (name, si, v)
+
+    def run(kind):
+        V, B = 24, 200
+        pa = port.Patch(d, V, delay_taps=taps, kind=kind)
+        for k, v in params(V, 11).items():
+            pa.set(k, v)
+        for blk in range(3):
+            o, m = pa.process(B, inputs(V, B, blk, 7), want_mix=True)
+            assert np.isfinite(o).all() and np.abs(o).max() > 1e-3
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+        for si, (op, kd, dst, src) in enumerate(d.stages):
+            for sl in range(SLOTS.get(op, 0)):
+                if op == 5 and kd in (5, 6) and sl == 1:
+                    continue                                   # lopass / hipass keep one value (outputs[0])
+                if op == 4 and sl == 3:
+                    continue                                   # nxcHappened is indeterminate in the reference until the first trigger
+                yield f"stage {si} slot {sl}", pa.get_state(si, sl)
+            if op in (10, 11):
+                for v in range(0, V, 5):
+                    yield f"stage {si} ring {v}", pa.ring(si, v, taps)
+    reference.check(run)
 
 
 @pytest.mark.parametrize("case", PC.cases(), ids=lambda c: c[0])
@@ -73,24 +81,28 @@ def test_chorus_port_equals_reference(port, reference):
     name, d, params, _, exact, taps = PC.chorus()
     V, B, NB, seed = 9, 150, 3, 777
     noise = port.noise_fill(seed, NB * B * V, "port").reshape(NB, B, V)
-    assert np.array_equal(noise, reference.noise_fill(seed, NB * B * V, "reference").reshape(NB, B, V))
     assert np.abs(noise).max() <= 1.0 and noise.std() > 0.5
-    po = port.Patch(d, V, delay_taps=taps, kind="port"); pr = reference.Patch(d, V, delay_taps=taps, kind="reference")
-    for k, v in params(V, 3).items():
-        po.set(k, v); pr.set(k, v)
-    reference.srand(seed, "reference")
     si = [i for i, st in enumerate(d.stages) if st[0] == 18][0]
-    for blk in range(NB):
-        orr, mr = pr.process(B, {"noise": noise[blk]}, want_mix=True)          # draws from rand() itself
-        oo, mo = po.process(B, {"noise": noise[blk]}, want_mix=True)
-        assert np.array_equal(oo, orr), blk
-        assert np.array_equal(mo, mr), blk
-        assert np.isfinite(orr).all() and np.abs(orr).max() > 1e-3
-    for sl in range(4):
-        assert np.array_equal(po.get_state(si, sl), pr.get_state(si, sl)), sl
-    for v in range(V):
-        assert np.array_equal(po.ring(si, v, 2 * taps), pr.ring(si, v, 2 * taps)), v
-    assert len({int(x) for x in po.get_state(si, 0)} | {int(x) for x in po.get_state(si, 1)}) > 2      # the lines are swept: indices diverged
+
+    def run(kind):
+        yield "noise", noise if kind == "port" else port.noise_fill(seed, NB * B * V, kind).reshape(NB, B, V)
+        pa = port.Patch(d, V, delay_taps=taps, kind=kind)
+        for k, v in params(V, 3).items():
+            pa.set(k, v)
+        if kind == "reference":
+            port.srand(seed, kind)
+        for blk in range(NB):
+            o, m = pa.process(B, {"noise": noise[blk]}, want_mix=True)     # the reference draws from rand() itself
+            assert np.isfinite(o).all() and np.abs(o).max() > 1e-3
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+        for sl in range(4):
+            yield f"slot {sl}", pa.get_state(si, sl)
+        for v in range(V):
+            yield f"ring {v}", pa.ring(si, v, 2 * taps)
+        if kind == "port":      # the lines are swept: indices diverged
+            assert len({int(x) for x in pa.get_state(si, 0)} | {int(x) for x in pa.get_state(si, 1)}) > 2
+    reference.check(run)
 
 
 def test_chorus_golden_exact(port):

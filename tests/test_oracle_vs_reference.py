@@ -1,7 +1,9 @@
 """Pins the plain-C oracle (oracle/maxi_oracle.c) BIT-FOR-BIT against the unmodified reference
-compiled from /root/reference (oracle/_ref/libmaxiref.so, built by oracle/Makefile).
+compiled by oracle/Makefile (oracle/_ref/libmaxiref.so).
 
-CPU only. Skipped when the compiled reference is neither present nor buildable (GPU box).
+CPU only. Each test drives one library through a scenario (run(kind)); the port's values must equal the
+reference's, live where the compiled reference is present and against its stored trace everywhere
+(tests/reference_trace.py).
 Tolerance: none. fp64 and fp32 values are compared with ==, integer state exactly.
 """
 import itertools
@@ -18,125 +20,135 @@ FILTS = ["none", "lores", "hires", "svf", "biquad"]
 _configure = W.configure_bank
 
 
-def _pair(port, reference, V, **kw):
-    return port.Bank(V, kind="port", **kw), reference.Bank(V, kind="reference", **kw)
-
-
 def _same(a, b):
     return np.array_equal(a, b, equal_nan=True)
 
 
 @pytest.mark.parametrize("osc,filt", list(itertools.product(OSCS, FILTS)))
 def test_osc_filter_chains_bit_exact(port, reference, osc, filt):
-    V, B = 37, 257
-    p = W.voice_params(V, seed=11)
-    a, b = _pair(port, reference, V, osc=osc, filt=filt)
-    _configure(a, filt, p, False, False); _configure(b, filt, p, False, False)
-    for _ in range(3):                        # state carried over consecutive blocks
-        oa, ma = a.process(B, want_mix=True)
-        ob, mb = b.process(B, want_mix=True)
-        assert _same(oa, ob)
-        assert _same(ma, mb)
-    for s in ("phase", "filt0", "filt1", "filt2"):
-        assert _same(a.get(s), b.get(s)), s
+    def run(kind):
+        V, B = 37, 257
+        p = W.voice_params(V, seed=11)
+        b = port.Bank(V, kind=kind, osc=osc, filt=filt)
+        _configure(b, filt, p, False, False)
+        for blk in range(3):                      # state carried over consecutive blocks
+            o, m = b.process(B, want_mix=True)
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+        for s in ("phase", "filt0", "filt1", "filt2"):
+            yield s, b.get(s)
+    reference.check(run)
 
 
 @pytest.mark.parametrize("btype", ["lowpass", "highpass", "bandpass", "notch", "peak", "lowshelf", "highshelf"])
 @pytest.mark.parametrize("gain_sign", [1.0, -1.0])
 def test_biquad_types_bit_exact(port, reference, btype, gain_sign):
-    V, B = 16, 300
-    p = W.voice_params(V, seed=5)
-    p["gain"] = gain_sign * (0.5 + 11.5 * np.random.default_rng(3).random(V))
-    a, b = _pair(port, reference, V, osc="saw", filt="biquad", biquad_type=btype)
-    _configure(a, "biquad", p, False, False); _configure(b, "biquad", p, False, False)
-    oa, _ = a.process(B); ob, _ = b.process(B)
-    assert _same(oa, ob)
+    def run(kind):
+        V, B = 16, 300
+        p = W.voice_params(V, seed=5)
+        p["gain"] = gain_sign * (0.5 + 11.5 * np.random.default_rng(3).random(V))
+        b = port.Bank(V, kind=kind, osc="saw", filt="biquad", biquad_type=btype)
+        _configure(b, "biquad", p, False, False)
+        yield "out", b.process(B)[0]
+    reference.check(run)
 
 
 @pytest.mark.parametrize("mix", [(1, 0, 0, 0), (0, 1, 0, 0), (0, 0, 1, 0), (0, 0, 0, 1), (0.3, 0.2, 0.4, 0.1)])
 def test_svf_mixes_bit_exact(port, reference, mix):
-    V, B = 16, 300
-    p = W.voice_params(V, seed=6)
-    p["res_svf"][0] = 0.0                     # res == 0 -> damping 0 branch (src/maximilian.h:1327)
-    a, b = _pair(port, reference, V, osc="saw", filt="svf", svf_mix=tuple(float(m) for m in mix))
-    _configure(a, "svf", p, False, False); _configure(b, "svf", p, False, False)
-    oa, _ = a.process(B); ob, _ = b.process(B)
-    assert _same(oa, ob)
+    def run(kind):
+        V, B = 16, 300
+        p = W.voice_params(V, seed=6)
+        p["res_svf"][0] = 0.0                     # res == 0 -> damping 0 branch (src/maximilian.h:1327)
+        b = port.Bank(V, kind=kind, osc="saw", filt="svf", svf_mix=tuple(float(m) for m in mix))
+        _configure(b, "svf", p, False, False)
+        yield "out", b.process(B)[0]
+    reference.check(run)
 
 
 def test_lores_clamps_bit_exact(port, reference):
     # cutoff < 10 -> 10, cutoff > sr -> sr (NaN: z == 1 gives 0/0), resonance < 1 -> 1  (SURVEY.md A3)
-    V, B = 6, 64
-    p = W.voice_params(V, seed=2)
-    p["cutoff"] = np.array([1.0, 9.999, 10.0, 47999.0, 48000.0, 96000.0])
-    p["q_lores"] = np.array([0.0, 0.5, 1.0, 1.5, 2.0, 3.0])
-    for filt in ("lores", "hires"):
-        a, b = _pair(port, reference, V, osc="saw", filt=filt)
-        _configure(a, filt, p, False, False); _configure(b, filt, p, False, False)
-        oa, _ = a.process(B); ob, _ = b.process(B)
-        assert _same(oa, ob)
-        assert np.isnan(oa[-1, 4]) and np.isnan(oa[-1, 5])
+    def run(kind):
+        V, B = 6, 64
+        p = W.voice_params(V, seed=2)
+        p["cutoff"] = np.array([1.0, 9.999, 10.0, 47999.0, 48000.0, 96000.0])
+        p["q_lores"] = np.array([0.0, 0.5, 1.0, 1.5, 2.0, 3.0])
+        for filt in ("lores", "hires"):
+            b = port.Bank(V, kind=kind, osc="saw", filt=filt)
+            _configure(b, filt, p, False, False)
+            o, _ = b.process(B)
+            if kind == "port":
+                assert np.isnan(o[-1, 4]) and np.isnan(o[-1, 5])
+            yield filt, o
+    reference.check(run)
 
 
 def test_sample_rates(port, reference):
-    for sr in (44100, 48000, 96000):
-        V, B = 8, 200
-        p = W.voice_params(V, seed=sr)
-        a, b = _pair(port, reference, V, osc="sinewave", filt="svf", sample_rate=sr)
-        _configure(a, "svf", p, False, False); _configure(b, "svf", p, False, False)
-        oa, _ = a.process(B); ob, _ = b.process(B)
-        assert _same(oa, ob)
+    def run(kind):
+        for sr in (44100, 48000, 96000):
+            V, B = 8, 200
+            p = W.voice_params(V, seed=sr)
+            b = port.Bank(V, kind=kind, osc="sinewave", filt="svf", sample_rate=sr)
+            _configure(b, "svf", p, False, False)
+            yield f"out {sr}", b.process(B)[0]
+    reference.check(run)
 
 
 @pytest.mark.parametrize("filt", ["none", "lores"])
 def test_env_state_machine_bit_exact(port, reference, filt):
-    V, B = 64, 512
-    p = W.voice_params(V, seed=9)
-    p["env_holdtime"] = np.array([1, 1, 0, 5, 100, 1000, 1, 3] * (V // 8), dtype=np.float64)
-    a, b = _pair(port, reference, V, osc="saw", filt=filt, env=True)
-    _configure(a, filt, p, True, False); _configure(b, filt, p, True, False)
-    for blk in range(8):
-        on, off = W.gate(V, B, blk)
-        if blk == 5:                          # retrigger while still releasing, gate across the whole block
-            on[:] = 0; off[:] = B
-        oa, _ = a.process(B, on, off); ob, _ = b.process(B, on, off)
-        assert _same(oa, ob), blk
-        for s in ("env_amplitude", "env_output", "env_holdcount", "env_flags"):
-            assert _same(a.get(s), b.get(s)), (blk, s)
+    def run(kind):
+        V, B = 64, 512
+        p = W.voice_params(V, seed=9)
+        p["env_holdtime"] = np.array([1, 1, 0, 5, 100, 1000, 1, 3] * (V // 8), dtype=np.float64)
+        b = port.Bank(V, kind=kind, osc="saw", filt=filt, env=True)
+        _configure(b, filt, p, True, False)
+        for blk in range(8):
+            on, off = W.gate(V, B, blk)
+            if blk == 5:                          # retrigger while still releasing, gate across the whole block
+                on[:] = 0; off[:] = B
+            yield f"out {blk}", b.process(B, on, off)[0]
+            for s in ("env_amplitude", "env_output", "env_holdcount", "env_flags"):
+                yield f"{s} {blk}", b.get(s)
+    reference.check(run)
 
 
 def test_env_setters(port, reference):
-    la, lb = port.load("port"), reference.load("reference")
-    for ms in (0.5, 1.0, 2.0, 17.3, 500.0):
-        for sr in (44100, 48000):
-            assert la.mxo_env_attack_coeff(ms, sr) == lb.mxo_env_attack_coeff(ms, sr)
-            assert la.mxo_env_attack_ms_coeff(ms, sr) == lb.mxo_env_attack_ms_coeff(ms, sr)
-            assert la.mxo_env_decay_coeff(ms, sr) == lb.mxo_env_decay_coeff(ms, sr)
-    p = W.voice_params(8, seed=1)
-    att, dec, rel = W.env_coeffs(p)           # math.pow == libm pow
-    for i in range(8):
-        assert att[i] == lb.mxo_env_attack_coeff(p["attack_ms"][i], 48000)
-        assert dec[i] == lb.mxo_env_decay_coeff(p["decay_ms"][i], 48000)
-        assert rel[i] == lb.mxo_env_decay_coeff(p["release_ms"][i], 48000)
+    def run(kind):
+        lib = port.load(kind)
+        for ms in (0.5, 1.0, 2.0, 17.3, 500.0):
+            for sr in (44100, 48000):
+                yield f"attack {ms} {sr}", lib.mxo_env_attack_coeff(ms, sr)
+                yield f"attack_ms {ms} {sr}", lib.mxo_env_attack_ms_coeff(ms, sr)
+                yield f"decay {ms} {sr}", lib.mxo_env_decay_coeff(ms, sr)
+        p = W.voice_params(8, seed=1)
+        if kind == "port":
+            att, dec, rel = W.env_coeffs(p)       # math.pow == libm pow
+        else:
+            att = [lib.mxo_env_attack_coeff(p["attack_ms"][i], 48000) for i in range(8)]
+            dec = [lib.mxo_env_decay_coeff(p["decay_ms"][i], 48000) for i in range(8)]
+            rel = [lib.mxo_env_decay_coeff(p["release_ms"][i], 48000) for i in range(8)]
+        for i in range(8):
+            yield f"env_coeffs {i}", np.array([att[i], dec[i], rel[i]], dtype=np.float64)
+    reference.check(run)
 
 
 def test_delayline_indices_and_ring_bit_exact(port, reference):
-    # small V: every reference maxiDelayline is a 5.6 MB object (src/maximilian.h:273)
-    V, B, cap = 12, 700, 512
-    p = W.voice_params(V, seed=4, delay_size=cap, ragged_delay=True)
-    p["delay_size"][:4] = [1, 2, 3, cap]
-    a, b = _pair(port, reference, V, osc="saw", env=True, delay=True, delay_capacity=cap)
-    _configure(a, "none", p, True, True); _configure(b, "none", p, True, True)
-    for blk in range(4):
-        on, off = W.gate(V, B, blk)
-        if blk == 2:                          # size shrinks mid-stream: phase >= size -> 0 on the next call (A6)
-            p["delay_size"] = np.maximum(1, p["delay_size"] // 2)
-            a.set("delay_size", p["delay_size"]); b.set("delay_size", p["delay_size"])
-        oa, _ = a.process(B, on, off); ob, _ = b.process(B, on, off)
-        assert _same(oa, ob), blk
-        assert np.array_equal(a.get("delay_phase"), b.get("delay_phase"))     # integer index: exact
-    for v in range(V):
-        assert _same(a.ring(v, cap), b.ring(v, cap)), v
+    def run(kind):
+        # small V: every reference maxiDelayline is a 5.6 MB object (src/maximilian.h:273)
+        V, B, cap = 12, 700, 512
+        p = W.voice_params(V, seed=4, delay_size=cap, ragged_delay=True)
+        p["delay_size"][:4] = [1, 2, 3, cap]
+        b = port.Bank(V, kind=kind, osc="saw", env=True, delay=True, delay_capacity=cap)
+        _configure(b, "none", p, True, True)
+        for blk in range(4):
+            on, off = W.gate(V, B, blk)
+            if blk == 2:                          # size shrinks mid-stream: phase >= size -> 0 on the next call (A6)
+                p["delay_size"] = np.maximum(1, p["delay_size"] // 2)
+                b.set("delay_size", p["delay_size"])
+            yield f"out {blk}", b.process(B, on, off)[0]
+            yield f"delay_phase {blk}", b.get("delay_phase")     # integer index: exact
+        for v in range(V):
+            yield f"ring {v}", b.ring(v, cap)
+    reference.check(run)
 
 
 def fm_frequencies(V, B, blk, seed=5):
@@ -149,16 +161,15 @@ def fm_frequencies(V, B, blk, seed=5):
 
 @pytest.mark.parametrize("osc,filt", [("sinewave", "none"), ("saw", "svf"), ("triangle", "lores")])
 def test_per_sample_frequency_bit_exact(port, reference, osc, filt):
-    V, B = 21, 200
-    p = W.voice_params(V, seed=31)
-    a, b = _pair(port, reference, V, osc=osc, filt=filt)
-    _configure(a, filt, p); _configure(b, filt, p)
-    for blk in range(3):
-        f = fm_frequencies(V, B, blk)
-        oa, _ = a.process(B, freq_tv=f); ob, _ = b.process(B, freq_tv=f)
-        assert _same(oa, ob), blk
-    oa, _ = a.process(B); ob, _ = b.process(B)          # back to the block-constant frequency
-    assert _same(oa, ob)
+    def run(kind):
+        V, B = 21, 200
+        p = W.voice_params(V, seed=31)
+        b = port.Bank(V, kind=kind, osc=osc, filt=filt)
+        _configure(b, filt, p)
+        for blk in range(3):
+            yield f"out {blk}", b.process(B, freq_tv=fm_frequencies(V, B, blk))[0]
+        yield "out block-constant", b.process(B)[0]           # back to the block-constant frequency
+    reference.check(run)
 
 
 def cutoff_sweeps(V, B, blk, seed=6):
@@ -172,26 +183,30 @@ def cutoff_sweeps(V, B, blk, seed=6):
 @pytest.mark.parametrize("osc,filt,fm", [("saw", "svf", False), ("saw", "lores", False), ("phasor", "hires", True), ("square", "svf", True)])
 def test_per_sample_cutoff_bit_exact(port, reference, osc, filt, fm):
     # lores/hires take the cutoff per call; the SVF patch calls setCutoff() per sample (src/maximilian.h:1287-1290)
-    V, B = 19, 160
-    p = W.voice_params(V, seed=33)
-    a, b = _pair(port, reference, V, osc=osc, filt=filt)
-    _configure(a, filt, p); _configure(b, filt, p)
-    for blk in range(3):
-        cu = cutoff_sweeps(V, B, blk); f = fm_frequencies(V, B, blk) if fm else None
-        oa, ma = a.process(B, freq_tv=f, cutoff_tv=cu, want_mix=True); ob, mb = b.process(B, freq_tv=f, cutoff_tv=cu, want_mix=True)
-        assert _same(oa, ob) and _same(ma, mb), blk
-    oa, _ = a.process(B); ob, _ = b.process(B)          # the block-constant cutoff is in force again
-    assert _same(oa, ob)
-    for s in ("filt0", "filt1"):
-        assert _same(a.get(s), b.get(s)), s
+    def run(kind):
+        V, B = 19, 160
+        p = W.voice_params(V, seed=33)
+        b = port.Bank(V, kind=kind, osc=osc, filt=filt)
+        _configure(b, filt, p)
+        for blk in range(3):
+            cu = cutoff_sweeps(V, B, blk); f = fm_frequencies(V, B, blk) if fm else None
+            o, m = b.process(B, freq_tv=f, cutoff_tv=cu, want_mix=True)
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+        yield "out block-constant", b.process(B)[0]           # the block-constant cutoff is in force again
+        for s in ("filt0", "filt1"):
+            yield s, b.get(s)
+    reference.check(run)
 
 
 def test_per_sample_cutoff_not_for_biquad(port, reference):
-    for lib in (port, reference):
-        bq = lib.Bank(4, osc="saw", filt="biquad")
+    def run(kind):
+        bq = port.Bank(4, osc="saw", filt="biquad", kind=kind)
         bq.set("cutoff", 800.0); bq.set("resonance", 1.0); bq.set("gain", 0.0)
         with pytest.raises(RuntimeError):
             bq.process(8, cutoff_tv=np.full((8, 4), 500.0))
+        yield "refused", True
+    reference.check(run)
 
 
 def flanger_sizes(V, B, blk, cap, seed=7):
@@ -207,69 +222,68 @@ def flanger_sizes(V, B, blk, cap, seed=7):
 
 @pytest.mark.parametrize("delay", ["dl", "position"])
 def test_per_sample_delay_size_bit_exact(port, reference, delay):
-    V, B, cap = 10, 300, 256            # small V: every reference maxiDelayline is a 5.6 MB object
-    p = W.voice_params(V, seed=41, delay_size=cap, ragged_delay=True)
-    a, b = _pair(port, reference, V, osc="saw", filt="lores", env=True, delay=delay, delay_capacity=cap)
-    _configure(a, "lores", p, True, True); _configure(b, "lores", p, True, True)
-    if delay == "position":
-        pos = np.arange(V, dtype=np.float64) * 3.0
-        a.set("delay_position", pos); b.set("delay_position", pos)
-    for blk in range(3):
-        on, off = W.gate(V, B, blk); sz = flanger_sizes(V, B, blk, cap)
-        oa, _ = a.process(B, on, off, delay_size_tv=sz); ob, _ = b.process(B, on, off, delay_size_tv=sz)
-        assert _same(oa, ob), blk
-        assert np.array_equal(a.get("delay_phase"), b.get("delay_phase"))
-    oa, _ = a.process(B); ob, _ = b.process(B)          # back to the block-constant size
-    assert _same(oa, ob)
-    for v in range(V):
-        assert _same(a.ring(v, cap), b.ring(v, cap)), v
+    def run(kind):
+        V, B, cap = 10, 300, 256            # small V: every reference maxiDelayline is a 5.6 MB object
+        p = W.voice_params(V, seed=41, delay_size=cap, ragged_delay=True)
+        b = port.Bank(V, kind=kind, osc="saw", filt="lores", env=True, delay=delay, delay_capacity=cap)
+        _configure(b, "lores", p, True, True)
+        if delay == "position":
+            b.set("delay_position", np.arange(V, dtype=np.float64) * 3.0)
+        for blk in range(3):
+            on, off = W.gate(V, B, blk)
+            yield f"out {blk}", b.process(B, on, off, delay_size_tv=flanger_sizes(V, B, blk, cap))[0]
+            yield f"delay_phase {blk}", b.get("delay_phase")
+        yield "out block-constant", b.process(B)[0]           # back to the block-constant size
+        for v in range(V):
+            yield f"ring {v}", b.ring(v, cap)
+    reference.check(run)
 
 
 def test_env_ar_bit_exact(port, reference):
     # maxiEnv::ar(input, attack, release, holdtime, trigger), src/maximilian.cpp:1319-1358
-    V, B = 48, 400
-    p = W.voice_params(V, seed=19)
-    att, dec, rel = W.env_coeffs(p)
-    hold = np.array([1, 0, 5, 50, 300, 1, 2, 1000] * (V // 8), dtype=np.float64)
-    a, b = _pair(port, reference, V, osc="saw", filt="lores", env="ar")
-    for k in (a, b):
-        _configure(k, "lores", p)
-        k.set("env_attack", att); k.set("env_release", rel); k.set("env_holdtime", hold)
-    for blk in range(6):
-        on, off = W.gate(V, B, blk)
-        if blk == 3:
-            on[:] = 0; off[:] = B
-        oa, _ = a.process(B, on, off); ob, _ = b.process(B, on, off)
-        assert _same(oa, ob), blk
-        for s in ("env_amplitude", "env_output", "env_holdcount", "env_flags"):
-            assert _same(a.get(s), b.get(s)), (blk, s)
+    def run(kind):
+        V, B = 48, 400
+        p = W.voice_params(V, seed=19)
+        att, dec, rel = W.env_coeffs(p)
+        hold = np.array([1, 0, 5, 50, 300, 1, 2, 1000] * (V // 8), dtype=np.float64)
+        b = port.Bank(V, kind=kind, osc="saw", filt="lores", env="ar")
+        _configure(b, "lores", p)
+        b.set("env_attack", att); b.set("env_release", rel); b.set("env_holdtime", hold)
+        for blk in range(6):
+            on, off = W.gate(V, B, blk)
+            if blk == 3:
+                on[:] = 0; off[:] = B
+            yield f"out {blk}", b.process(B, on, off)[0]
+            for s in ("env_amplitude", "env_output", "env_holdcount", "env_flags"):
+                yield f"{s} {blk}", b.get(s)
+    reference.check(run)
 
 
 def test_dl_from_position_bit_exact(port, reference):
     # maxiDelayline::dlFromPosition, src/maximilian.cpp:431-439
-    V, B, cap = 10, 300, 256
-    p = W.voice_params(V, seed=23, delay_size=cap, ragged_delay=True)
-    pos = np.array([0, 1, 5, 63, 64, 100, 200, 255, 300, 17], dtype=np.float64)     # 300 >= size -> 0
-    a, b = _pair(port, reference, V, osc="saw", delay="position", delay_capacity=cap)
-    for k in (a, b):
-        _configure(k, "none", p, False, True)
-        k.set("delay_position", pos)
-    for blk in range(3):
-        oa, _ = a.process(B); ob, _ = b.process(B)
-        assert _same(oa, ob), blk
-        assert np.array_equal(a.get("delay_phase"), b.get("delay_phase"))
-    for v in range(V):
-        assert _same(a.ring(v, cap), b.ring(v, cap)), v
+    def run(kind):
+        V, B, cap = 10, 300, 256
+        p = W.voice_params(V, seed=23, delay_size=cap, ragged_delay=True)
+        pos = np.array([0, 1, 5, 63, 64, 100, 200, 255, 300, 17], dtype=np.float64)     # 300 >= size -> 0
+        b = port.Bank(V, kind=kind, osc="saw", delay="position", delay_capacity=cap)
+        _configure(b, "none", p, False, True)
+        b.set("delay_position", pos)
+        for blk in range(3):
+            yield f"out {blk}", b.process(B)[0]
+            yield f"delay_phase {blk}", b.get("delay_phase")
+        for v in range(V):
+            yield f"ring {v}", b.ring(v, cap)
+    reference.check(run)
 
 
 def test_delay_size_nonpositive(port, reference):
-    V, B = 3, 20
-    a, b = _pair(port, reference, V, osc="saw", delay=True, delay_capacity=16)
-    for k in (a, b):
-        k.set("freq", [100.0, 200.0, 300.0]); k.set("delay_size", [0.0, -3.0, 1.0]); k.set("delay_feedback", 0.7)
-    oa, _ = a.process(B); ob, _ = b.process(B)
-    assert _same(oa, ob)
-    assert np.array_equal(a.get("delay_phase"), b.get("delay_phase"))
+    def run(kind):
+        V, B = 3, 20
+        b = port.Bank(V, kind=kind, osc="saw", delay=True, delay_capacity=16)
+        b.set("freq", [100.0, 200.0, 300.0]); b.set("delay_size", [0.0, -3.0, 1.0]); b.set("delay_feedback", 0.7)
+        yield "out", b.process(B)[0]
+        yield "delay_phase", b.get("delay_phase")
+    reference.check(run)
 
 
 def test_threaded_partition_matches_serial(port):
@@ -287,19 +301,20 @@ def test_threaded_partition_matches_serial(port):
 
 @pytest.mark.parametrize("n,hop", [(1024, 512), (1024, 256), (512, 128), (256, 256), (64, 16)])
 def test_stft_bit_exact(port, reference, n, hop):
-    C = 5
-    x = W.channel_streams(C, 6 * n + 37, seed=n + hop)
-    x[1] *= 1000.0
-    x[2] = 0.0
-    a = port.Stft(C, n, hop, kind="port"); b = reference.Stft(C, n, hop, kind="reference")
-    assert _same(a.window(), b.window())
-    # feed in uneven chunks: the frame schedule (integer pos) must agree exactly
-    cuts = [0, 3, hop - 1, hop, 2 * n + 5, x.shape[1]]
-    for lo, hi in zip(cuts[:-1], cuts[1:]):
-        ra = a.process(x[:, lo:hi]); rb = b.process(x[:, lo:hi])
-        assert ra["mags"].shape == rb["mags"].shape
-        for k in ("re", "im", "mags", "phases"):
-            assert _same(ra[k], rb[k]), (k, lo, hi)
+    def run(kind):
+        C = 5
+        x = W.channel_streams(C, 6 * n + 37, seed=n + hop)
+        x[1] *= 1000.0
+        x[2] = 0.0
+        s = port.Stft(C, n, hop, kind=kind)
+        yield "window", s.window()
+        # feed in uneven chunks: the frame schedule (integer pos) must agree exactly
+        cuts = [0, 3, hop - 1, hop, 2 * n + 5, x.shape[1]]
+        for lo, hi in zip(cuts[:-1], cuts[1:]):
+            r = s.process(x[:, lo:hi])
+            for k in ("re", "im", "mags", "phases"):
+                yield f"{k} {lo}:{hi}", r[k]
+    reference.check(run)
 
 
 def test_stft_frame_schedule(port):
@@ -319,11 +334,14 @@ def test_mfcc_bit_exact(port, reference, cfg):
     st = port.Stft(3, 2 * bins, bins)
     mags = st.process(W.channel_streams(3, 2 * bins * 8, seed=bins))["mags"]
     mags[0, 0] = 0.0                                   # silent frame: log gate (> 1e-6) takes the 0 branch
-    a = port.Mfcc(*cfg, kind="port"); b = reference.Mfcc(*cfg, kind="reference")
-    ca, ma = a.process(mags); cb, mb = b.process(mags)
-    assert _same(ma, mb)
-    assert _same(ca, cb)
-    assert np.all(ma[..., 0] == 0.0)                   # filter 0 is never initialised by the reference (A13)
+
+    def run(kind):
+        c, m = port.Mfcc(*cfg, kind=kind).process(mags)
+        if kind == "port":
+            assert np.all(m[..., 0] == 0.0)            # filter 0 is never initialised by the reference (A13)
+        yield "melbands", m
+        yield "coeffs", c
+    reference.check(run)
 
 
 def test_spectral_features_bit_exact(port, reference):
@@ -331,11 +349,12 @@ def test_spectral_features_bit_exact(port, reference):
     mags = port.Stft(3, 1024, 512).process(W.channel_streams(3, 8192, seed=8))["mags"]
     mags[0, 0] = 0.0                                  # all-zero frame: both features return 0
     mags[1, 1, :7] = 0.0                              # zeros are skipped by the geometric mean
-    for sr in (44100, 48000):
-        a = port.spectral_features(mags, 1024, sr, kind="port")
-        b = reference.spectral_features(mags, 1024, sr, kind="reference")
-        for x, y in zip(a, b):
-            assert _same(x, y)
+
+    def run(kind):
+        for sr in (44100, 48000):
+            for name, x in zip(("db", "flatness", "centroid"), port.spectral_features(mags, 1024, sr, kind=kind)):
+                yield f"{name} {sr}", x
+    reference.check(run)
 
 
 @pytest.mark.parametrize("n,hop", [(1024, 512), (1024, 256), (256, 64)])
@@ -343,12 +362,13 @@ def test_istft_bit_exact(port, reference, n, hop):
     C = 3
     x = W.channel_streams(C, 10 * n, seed=77)
     r = port.Stft(C, n, hop).process(x)
-    a = port.Istft(C, n, hop, kind="port"); b = reference.Istft(C, n, hop, kind="reference")
-    F = r["mags"].shape[1]
-    for lo, hi in ((0, 3), (3, F)):
-        ya = a.process(r["mags"][:, lo:hi], r["phases"][:, lo:hi])
-        yb = b.process(r["mags"][:, lo:hi], r["phases"][:, lo:hi])
-        assert _same(ya, yb)
+
+    def run(kind):
+        s = port.Istft(C, n, hop, kind=kind)
+        F = r["mags"].shape[1]
+        for lo, hi in ((0, 3), (3, F)):
+            yield f"y {lo}:{hi}", s.process(r["mags"][:, lo:hi], r["phases"][:, lo:hi])
+    reference.check(run)
 
 
 # ---- maxiFFTOctaveAnalyzer / maxiBark (SURVEY.md 8f-3) ------------------------------------------------------------------------
@@ -359,12 +379,17 @@ def test_octave_analyser_port_equals_reference(port, reference, per_octave, sr):
     calls), with the public members changed from their defaults: averages and peaks bit for bit."""
     x = W.channel_streams(3, 1024 * 9, seed=5)
     mags = port.Stft(3, 1024, 512, kind="port").process(x)["mags"]
-    a = port.Octave(3, sr, 512, per_octave, kind="port"); b = reference.Octave(3, sr, 512, per_octave, kind="reference")
-    assert a.n_averages == b.n_averages > 0
-    a.config(2, 0.8, 1.0, 0.01); b.config(2, 0.8, 1.0, 0.01)
-    for lo, hi in ((0, 5), (5, mags.shape[1])):
-        ra = a.process(mags[:, lo:hi]); rb = b.process(mags[:, lo:hi])
-        assert np.array_equal(ra[0], rb[0]) and np.array_equal(ra[1], rb[1]), (lo, hi)
+
+    def run(kind):
+        a = port.Octave(3, sr, 512, per_octave, kind=kind)
+        assert a.n_averages > 0
+        yield "n_averages", a.n_averages
+        a.config(2, 0.8, 1.0, 0.01)
+        for lo, hi in ((0, 5), (5, mags.shape[1])):
+            av, pk = a.process(mags[:, lo:hi])
+            yield f"averages {lo}:{hi}", av
+            yield f"peaks {lo}:{hi}", pk
+    reference.check(run)
 
 
 @pytest.mark.parametrize("sr,bs", [(48000, 1024), (44100, 1024), (48000, 512), (22050, 256)])
@@ -374,29 +399,34 @@ def test_bark_port_equals_reference(port, reference, sr, bs):
     turns into a crash)."""
     x = W.channel_streams(3, 1024 * 9, seed=6)
     mags = np.ascontiguousarray(port.Stft(3, 1024, 512, kind="port").process(x)["mags"][..., :bs // 2])
-    pa = port.bark(mags, sr, bs, "port"); pb = reference.bark(mags, sr, bs, "reference")
-    for u, v in zip(pa, pb):
-        assert np.array_equal(u, v, equal_nan=True)
+    pa = port.bark(mags, sr, bs, "port")
     assert np.all(pa[1].max(axis=-1) == 1.0)
+
+    def run(kind):
+        for name, u in zip(("specific", "relative", "total"), pa if kind == "port" else port.bark(mags, sr, bs, kind)):
+            yield name, u
+    reference.check(run)
 
 
 @pytest.mark.parametrize("filt,delay,env", [("none", False, "adsr"), ("lores", False, "ar"), ("svf", True, "adsr")])
 def test_per_sample_trigger_port_equals_reference(port, reference, filt, delay, env):
     """maxiEnv::trigger written on every sample (mxo_bank_process_mod2): several notes per block, both envelope kinds."""
-    rng = np.random.default_rng(5)
-    V, B, cap = 12, 400, 64
-    p = W.voice_params(V, seed=61, delay_size=cap, ragged_delay=True)
-    a = port.Bank(V, osc="saw", filt=filt, env=env, delay=delay, delay_capacity=cap, kind="port")
-    b = reference.Bank(V, osc="saw", filt=filt, env=env, delay=delay, delay_capacity=cap, kind="reference")
-    W.configure_bank(a, filt, p, env=True, delay=delay); W.configure_bank(b, filt, p, env=True, delay=delay)
-    for blk in range(3):
-        tv = (rng.random((B, V)) < 0.5).astype(np.uint8)
-        tv[:, 0] = 0; tv[:, 1] = 1
-        tv[100:250, 2:6] = 1; tv[250:260, 2:6] = 0; tv[260:300, 2:6] = 1
-        oa, ma = a.process(B, trig_tv=tv, want_mix=True); ob, mb = b.process(B, trig_tv=tv, want_mix=True)
-        assert np.array_equal(oa, ob) and np.array_equal(ma, mb), blk
-        for s_ in ("env_holdcount", "env_flags", "env_amplitude", "env_output"):
-            assert np.array_equal(a.get(s_), b.get(s_)), (blk, s_)
+    def run(kind):
+        rng = np.random.default_rng(5)
+        V, B, cap = 12, 400, 64
+        p = W.voice_params(V, seed=61, delay_size=cap, ragged_delay=True)
+        b = port.Bank(V, osc="saw", filt=filt, env=env, delay=delay, delay_capacity=cap, kind=kind)
+        W.configure_bank(b, filt, p, env=True, delay=delay)
+        for blk in range(3):
+            tv = (rng.random((B, V)) < 0.5).astype(np.uint8)
+            tv[:, 0] = 0; tv[:, 1] = 1
+            tv[100:250, 2:6] = 1; tv[250:260, 2:6] = 0; tv[260:300, 2:6] = 1
+            o, m = b.process(B, trig_tv=tv, want_mix=True)
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+            for s_ in ("env_holdcount", "env_flags", "env_amplitude", "env_output"):
+                yield f"{s_} {blk}", b.get(s_)
+    reference.check(run)
 
 
 @pytest.mark.parametrize("osc,filt,env,cm,dsz", [("saw", "none", True, False, False), ("saw", "lores", True, True, False), ("pulse", "svf", False, True, False),
@@ -405,24 +435,25 @@ def test_modulated_chain_with_a_delay_line_port_equals_reference(port, reference
     """Per-sample frequency / cutoff (/ delay size / trigger) on a chain that ends in maxiDelayline::dl -- the combinations the modulated
     instantiation of K2 is tested against (tests/test_gpu_bank.py::test_modulated_frequency_and_cutoff_with_a_delay_line compares it
     with the port): the port itself against the compiled reference, samples, ring index and ring contents bit for bit."""
-    V, B, cap = 23, 150, 96
-    p = W.voice_params(V, seed=61, delay_size=cap, ragged_delay=True)
-    a, b = _pair(port, reference, V, osc=osc, filt=filt, env=env, delay=True, delay_capacity=cap)
-    _configure(a, filt, p, env, True); _configure(b, filt, p, env, True)
-    rng = np.random.default_rng(8)
-    for blk in range(3):
-        f = fm_frequencies(V, B, blk); cu = cutoff_sweeps(V, B, blk) if cm else None
-        tv = (rng.random((B, V)) < 0.4).astype(np.uint8) if env else None
-        sz = np.floor(1 + (cap - 1) * rng.random((B, V))) if dsz else None
-        oa, ma = a.process(B, freq_tv=f, cutoff_tv=cu, trig_tv=tv, delay_size_tv=sz, want_mix=True)
-        ob, mb = b.process(B, freq_tv=f, cutoff_tv=cu, trig_tv=tv, delay_size_tv=sz, want_mix=True)
-        assert _same(oa, ob) and _same(ma, mb), blk
-        assert _same(a.get("delay_phase"), b.get("delay_phase")), blk
-    on, off = (W.gate(V, B, 3) if env else (None, None))
-    oa, _ = a.process(B, on, off); ob, _ = b.process(B, on, off)
-    assert _same(oa, ob)
-    for v in (0, V // 2, V - 1):
-        assert _same(a.ring(v, cap), b.ring(v, cap)), v
+    def run(kind):
+        V, B, cap = 23, 150, 96
+        p = W.voice_params(V, seed=61, delay_size=cap, ragged_delay=True)
+        b = port.Bank(V, kind=kind, osc=osc, filt=filt, env=env, delay=True, delay_capacity=cap)
+        _configure(b, filt, p, env, True)
+        rng = np.random.default_rng(8)
+        for blk in range(3):
+            f = fm_frequencies(V, B, blk); cu = cutoff_sweeps(V, B, blk) if cm else None
+            tv = (rng.random((B, V)) < 0.4).astype(np.uint8) if env else None
+            sz = np.floor(1 + (cap - 1) * rng.random((B, V))) if dsz else None
+            o, m = b.process(B, freq_tv=f, cutoff_tv=cu, trig_tv=tv, delay_size_tv=sz, want_mix=True)
+            yield f"out {blk}", o
+            yield f"mix {blk}", m
+            yield f"delay_phase {blk}", b.get("delay_phase")
+        on, off = (W.gate(V, B, 3) if env else (None, None))
+        yield "out gated", b.process(B, on, off)[0]
+        for v in (0, V // 2, V - 1):
+            yield f"ring {v}", b.ring(v, cap)
+    reference.check(run)
 
 
 def test_per_sample_analysis_resynthesis_idiom(port, reference):
@@ -431,17 +462,26 @@ def test_per_sample_analysis_resynthesis_idiom(port, reference):
     compose them (tests/test_cpp_dropin.py::test_per_sample_feature_extractor_matches_oracle): a frame fires on the last sample of every
     hop; the resynthesis reads zeros during the first hop and frame k - 1 during hop k. Bit for bit."""
     import ctypes as C
-    lib = reference.load("reference")
-    fn = lib.mxo_ref_per_sample_roundtrip
-    fn.restype = C.c_int32
-    fn.argtypes = [C.POINTER(C.c_float), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_uint8)]
     N, n, hop, bins = 6 * 1024 + 300, 1024, 512, 512
     x = W.channel_streams(1, N, seed=45)
-    y = np.empty(N, dtype=np.float32); fired = np.empty(N, dtype=np.uint8)
-    F = fn(x.ctypes.data_as(C.POINTER(C.c_float)), N, n, hop, y.ctypes.data_as(C.POINTER(C.c_float)), fired.ctypes.data_as(C.POINTER(C.c_uint8)))
-    assert F == N // hop and np.array_equal(np.nonzero(fired)[0], hop * np.arange(1, F + 1) - 1)
-    o = port.Stft(1, n, hop, kind="port").process(x)
-    K = (N + hop - 1) // hop
-    z = np.zeros((1, 1, bins), dtype=np.float32)
-    oy = port.Istft(1, n, hop, kind="port").process(np.concatenate([z, o["mags"][:, :K - 1]], axis=1), np.concatenate([z, o["phases"][:, :K - 1]], axis=1))
-    assert np.array_equal(y, oy[0, :N])
+
+    def run(kind):
+        if kind == "reference":
+            fn = port.load("reference").mxo_ref_per_sample_roundtrip
+            fn.restype = C.c_int32
+            fn.argtypes = [C.POINTER(C.c_float), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_uint8)]
+            y = np.empty(N, dtype=np.float32); fired = np.empty(N, dtype=np.uint8)
+            F = fn(x.ctypes.data_as(C.POINTER(C.c_float)), N, n, hop, y.ctypes.data_as(C.POINTER(C.c_float)), fired.ctypes.data_as(C.POINTER(C.c_uint8)))
+            yield "frames", F
+            yield "fired", np.nonzero(fired)[0]
+            yield "y", y
+            return
+        F = N // hop
+        yield "frames", F
+        yield "fired", hop * np.arange(1, F + 1) - 1
+        o = port.Stft(1, n, hop, kind="port").process(x)
+        K = (N + hop - 1) // hop
+        z = np.zeros((1, 1, bins), dtype=np.float32)
+        oy = port.Istft(1, n, hop, kind="port").process(np.concatenate([z, o["mags"][:, :K - 1]], axis=1), np.concatenate([z, o["phases"][:, :K - 1]], axis=1))
+        yield "y", oy[0, :N]
+    reference.check(run)
